@@ -54,6 +54,9 @@ def parse():
     ap.add_argument("--no-shim-leg", action="store_true", help="skip the reference-host-with-GPU-shim point (64 files through oracle/_ref/jref_gpu)")
     ap.add_argument("--no-extra-legs", action="store_true", help="skip the 1-utterance / 16-utterance points and the short DNN-HMM leg")
     ap.add_argument("--cpu-sample-utts", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps write what the last timed step returned (pass-1 results of every utterance, "
+                         "word trellis of a fixed sample of utterances) as DIR/<name>.npy, to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -322,10 +325,50 @@ def fp32_peak():
 # 1.446 M with 32 (one launch per batch at 592 utterances: 1.357 M)
 PIPE_FRAMES_DEFAULT = 32
 
+# --dump-outputs: the trellises of this many utterances, drawn with a fixed seed, and no more than this many bytes in all
+DUMP_TRELLIS_UTTS = 64
+DUMP_SEED = 2024
+DUMP_MAX_BYTES = 64 << 20
 
-def measure_workload(ctx, name, B, T, steps, warmup, mode="exact", want_e2e=True, n_batches=2, seed0=100, pipe_frames=0):
+
+def dump_outputs(out_dir: str, res: list) -> None:
+    """Write the results of one decoded batch as float arrays, one .npy file each:
+    status, overflow, n_frames, score              [n_utts]   pass-1 result of every utterance
+    words, words_offset                            best word ids, concatenated; utterance u owns words[off[u]:off[u+1]]
+    trellis_utts, trellis_offset, trellis_<field>  word trellis (atoms) of a fixed, seeded sample of utterances
+    Integers are stored as float64, which holds every int32 exactly; scores stay float32."""
+    from julius_b200 import capi
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(res)
+    arrays = {
+        "status": np.array([r["status"] for r in res], np.float64),
+        "overflow": np.array([r["overflow"] for r in res], np.float64),
+        "n_frames": np.array([r["n_frames"] for r in res], np.float64),
+        "score": np.array([r["score"] for r in res], np.float32),
+        "words": np.array([w for r in res for w in r["words"]], np.float64),
+        "words_offset": np.cumsum([0] + [len(r["words"]) for r in res]).astype(np.float64),
+    }
+    pick = np.sort(np.random.default_rng(DUMP_SEED).permutation(n)[:DUMP_TRELLIS_UTTS])
+    bytes_per_atom = 4 * 8 + 2 * 4
+    budget = DUMP_MAX_BYTES - sum(a.nbytes for a in arrays.values()) - 8 * 2 * (len(pick) + 1)
+    while len(pick) and bytes_per_atom * sum(len(res[i]["atoms"]) for i in pick) > budget:
+        pick = pick[:-1]
+    atoms = [res[i]["atoms"] for i in pick]
+    cat = np.concatenate(atoms) if atoms else np.zeros(0, capi.ATOM_DT)
+    arrays["trellis_utts"] = pick.astype(np.float64)
+    arrays["trellis_offset"] = np.cumsum([0] + [len(a) for a in atoms]).astype(np.float64)
+    for k in ("wid", "begin", "end", "last"):
+        arrays["trellis_" + k] = cat[k].astype(np.float64)
+    for k in ("backscore", "lscore"):
+        arrays["trellis_" + k] = cat[k].astype(np.float32)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def measure_workload(ctx, name, B, T, steps, warmup, mode="exact", want_e2e=True, n_batches=2, seed0=100, pipe_frames=0,
+                     dump_dir=""):
     """W warm-up + K timed steps of one workload at B utterances x T frames per GPU; returns the measured figures.
-    ctx: dict(rank, local, world, device, torch, dist)."""
+    ctx: dict(rank, local, world, device, torch, dist).  dump_dir: where rank 0 writes the results of the last timed step."""
     torch, dist = ctx["torch"], ctx["dist"]
     from julius_b200 import capi, desc, workload
     from julius_b200.dist import broadcast_blob
@@ -413,6 +456,11 @@ def measure_workload(ctx, name, B, T, steps, warmup, mode="exact", want_e2e=True
     dev_ms = sum(score_ms) + sum(beam_ms)
     barrier()
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if dump_dir and rank == 0:
+        # the device path leaves its results in HBM: copy the last timed step's results to the host, as a caller would
+        capi._check(lib.jb200_decoder_fetch(dec.handle_ptr()), "decoder_fetch")
+        dec._last_n = B
+        dump_outputs(dump_dir, dec.results())
 
     # ---------------- e2e: host buffers through the C-ABI ----------------
     e2e_ms = h2d = d2h = 0
@@ -596,7 +644,8 @@ def product_main(a):
     ctx = dict(rank=rank, local=local, world=world, device=device, torch=torch, dist=dist)
 
     pf = PIPE_FRAMES_DEFAULT if a.pipe_frames < 0 else a.pipe_frames
-    r = measure_workload(ctx, a.workload, a.utts, a.frames, a.steps, a.warmup, mode=a.mode, pipe_frames=pf)
+    r = measure_workload(ctx, a.workload, a.utts, a.frames, a.steps, a.warmup, mode=a.mode, pipe_frames=pf,
+                         dump_dir=a.dump_outputs)
     B, T = r["B"], r["T"]
     extra = {}
     if world == 1 and not a.no_extra_legs:

@@ -5,8 +5,8 @@ import os
 import numpy as np
 import pytest
 
-from julius_b200 import capi, desc, refdump, workload
-from util import atoms_equal
+from julius_b200 import capi, desc, workload
+from util import GOLDEN, atoms_equal, load_pinned
 
 pytestmark = pytest.mark.gpu
 
@@ -47,10 +47,10 @@ def test_full_size_end_to_end_vs_oracle(full, oracle_lib):
 
 
 def test_probe_utterance_matches_compiled_reference(full):
-    """workloads/tri20k/probe.* was decoded by the compiled reference when the workload was built."""
-    u = refdump.load_refdump(workload.path(NAME, "probe.jrf"))[0]
+    """workloads/tri20k/probe.mfc, as the compiled reference decoded it (tests/golden/host/tri20k_probe)."""
     from julius_b200 import synth
     x, _ = synth.read_htk_param(workload.path(NAME, "probe.mfc"))
+    u = load_pinned(os.path.join(GOLDEN, "host", "tri20k_probe"), [x])[1][0]
     r = full["dec"].decode([x])[0]
     ok, why = atoms_equal(r["atoms"], u.atoms)
     assert ok, why

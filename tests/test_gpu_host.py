@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 from julius_b200 import refdump, synth
-from util import Golden, atoms_equal
+from util import GOLDEN, Golden, atoms_equal, digest, load_pinned
 
 pytestmark = pytest.mark.gpu
 
@@ -64,6 +64,11 @@ def _results(out):
     return [ln for ln in out.splitlines() if ln.startswith("JREF_RESULT")]
 
 
+def _stock(name):
+    """lines the stock host printed for the same run (tests/golden/make_golden.py)"""
+    return open(os.path.join(GOLDEN, "host", name)).read().splitlines()
+
+
 @pytest.mark.parametrize("case", ["small_b100", "small_iwsp"])
 def test_full_two_pass_recognition_is_unchanged_by_either_boundary(case, tmp_path):
     """SURVEY 8(f).1: the stock host runs BOTH passes; pass 2 (stack decoding on the word trellis,
@@ -71,8 +76,7 @@ def test_full_two_pass_recognition_is_unchanged_by_either_boundary(case, tmp_pat
     (a) the GPU fills the score cache, (b) the GPU beam builds the trellis, (c) both."""
     from oracle import ffi
     g, d, files = _prepare(case, tmp_path)
-    _, stock = ffi.run_ref(d, files, extra_args=g.meta["extra_args"], two_pass=True, dump="stock.jrf")
-    want = _results(stock)
+    want = _stock(f"{case}_two_pass.txt")
     assert len(want) == len(files) and all("sent0=" in w for w in want[:2])
     _, a = ffi.run_ref(d, files, extra_args=g.meta["extra_args"], two_pass=True, dump="a.jrf", env_extra={"JB200_ATTACH": "1"})
     assert _results(a) == want
@@ -91,12 +95,12 @@ def test_calcmix_hook_equals_gprune_none(tmp_path):
     from the GPU (jb200_gmm_gauss_host).  No pruning is applied, so the run must equal stock `-gprune none`."""
     from oracle import ffi
     g, d, files = _prepare("tiny", tmp_path)
-    dump0, _ = ffi.run_ref(d, files, extra_args=["-gprune", "none"], dump="none.jrf")
+    _, want = load_pinned(os.path.join(GOLDEN, "host", "tiny_gprune_none"), g.feats)      # the stock host, -gprune none
     dump1, out = ffi.run_ref(d, files, extra_args=["-gprune", "jb200"], dump="hook.jrf", env_extra={"JB200_ATTACH": "calcmix"})
-    want, got = refdump.load_refdump(dump0), refdump.load_refdump(dump1)
+    got = refdump.load_refdump(dump1)
     assert len(want) == len(got) == len(files)
     for u, v in zip(want, got):
-        assert np.array_equal(u.outprob.view(np.uint32), v.outprob.view(np.uint32))
+        assert digest(v.outprob) == u.outprob_sha256
         ok, why = atoms_equal(v.atoms, u.atoms)
         assert ok, why
         assert u.words == v.words and np.float32(u.score) == np.float32(v.score)
@@ -162,8 +166,7 @@ def test_progressive_output_matches_the_stock_host(case, tmp_path):
     from oracle import ffi
     g, d, files = _prepare(case, tmp_path)
     extra = g.meta["extra_args"] + ["-progout", "-proginterval", "100"]
-    _, stock = ffi.run_ref(d, files, extra_args=extra, dump="stock.jrf", env_extra={"JREF_INTERIM": "1"})
-    want = [ln for ln in stock.splitlines() if ln.startswith("JREF_INTERIM")]
+    want = _stock(f"{case}_interim.txt")
     assert len(want) >= 10 * len(files) and any("words=0," in w for w in want)
     dump, out = ffi.run_ref(d, files, extra_args=extra, binary=ffi.JREF_GPU, env_extra={"JREF_INTERIM": "1"})
     got = [ln for ln in out.splitlines() if ln.startswith("JREF_INTERIM")]

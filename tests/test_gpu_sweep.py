@@ -1,57 +1,40 @@
 """GPU: the CUDA path against the compiled reference across jconf options beyond the committed golden cases --
-the device-side twin of tests/test_oracle_sweep.py.  Each case samples fresh utterances, pushes them through the
-compiled reference (oracle/_ref/jref, which travels with the tree) and through K1 + K3, and demands bit-identical
-state scores and an identical word trellis.  Covers -iwcd1 avg / best N, -lmp, score-envelope pruning (-bs),
--gprune heuristic, -iwsp, transparent words, flattened tied-mixture codebooks and DFA grammars on the device."""
-import os
-
+the device-side twin of tests/test_oracle_sweep.py.  Each case's inputs go through K1 + K3 and must give the state
+scores (bit for bit) and the word trellis the compiled reference produced for them (tests/golden/sweep).  Covers
+-iwcd1 avg / best N, -lmp, score-envelope pruning (-bs), -gprune heuristic, -iwsp, transparent words, flattened
+tied-mixture codebooks and DFA grammars on the device."""
 import numpy as np
 import pytest
 
-from julius_b200 import capi, desc, refdump, synth
-from util import ROOT, atoms_equal
-from test_oracle_sweep import SWEEP, GRAMMAR_SWEEP
+from julius_b200 import capi
+from util import GRAMMAR_SWEEP, SWEEP, SweepGolden, atoms_equal, digest
 
 pytestmark = pytest.mark.gpu
-JREF = os.path.join(ROOT, "oracle", "_ref", "jref")
 
 
 def _check(r, u):
     ok, why = atoms_equal(r["atoms"], u.atoms)
     assert ok, why
     assert r["words"] == u.words and r["status"] == u.status and r["overflow"] == 0
-    assert np.float32(r["score"]) == np.float32(u.score)
+    assert np.float32(r["score"]) == u.score
 
 
-@pytest.mark.skipif(not os.path.exists(JREF), reason="compiled reference (oracle/_ref/jref) not present")
-@pytest.mark.parametrize("preset,extra", SWEEP, ids=[" ".join([p] + e) for p, e in SWEEP])
-def test_gpu_path_equals_compiled_reference(preset, extra, tmp_path):
-    from oracle import fixtures
-    d = str(tmp_path)
-    m, files, dump, out = fixtures.make_fixture(preset, d, n_utts=2, n_frames=150, extra_args=extra, noise_utts=1)
-    ds = desc.Descriptors(refdump.load_blob(os.path.join(d, "model.jb2m")))
-    utts = refdump.load_refdump(dump)
-    feats = [synth.read_htk_param(fn)[0] for fn in files]
-    am = capi.GmmScorer(ds, mode=capi.GMM_EXACT)
-    for u, x in zip(utts, feats):
+def _check_case(g):
+    am = capi.GmmScorer(g.ds, mode=capi.GMM_EXACT)
+    for u, x in zip(g.utts, g.feats):
         sc = am.score(x)
-        assert np.array_equal(sc.view(np.uint32), u.outprob.view(np.uint32)), "state scores differ from the reference"
-    dec = capi.Decoder(ds, am, max_utts=4, max_frames=2048)
-    for r, u in zip(dec.decode(feats), utts):
+        assert digest(sc) == u.outprob_sha256, "state scores differ from the reference"
+    dec = capi.Decoder(g.ds, am, max_utts=4, max_frames=2048)
+    for r, u in zip(dec.decode(g.feats), g.utts):
         _check(r, u)
+
+
+@pytest.mark.parametrize("preset,extra", SWEEP, ids=[" ".join([p] + e) for p, e in SWEEP])
+def test_gpu_path_equals_compiled_reference(preset, extra):
+    _check_case(SweepGolden(preset, extra))
 
 
 # the GPU beam takes grammars on normal trees only (creation refuses -multipath loudly, tested in test_gpu_beam.py)
-@pytest.mark.skipif(not os.path.exists(JREF), reason="compiled reference (oracle/_ref/jref) not present")
 @pytest.mark.parametrize("extra", [e for e in GRAMMAR_SWEEP if "-multipath" not in e], ids=lambda e: " ".join(e))
-def test_gpu_grammar_mode_equals_compiled_reference(extra, tmp_path):
-    from oracle import fixtures
-    d = str(tmp_path)
-    m, files, dump, out = fixtures.make_fixture("small", d, n_utts=2, n_frames=180, extra_args=extra, noise_utts=1, grammar=True)
-    ds = desc.Descriptors(refdump.load_blob(os.path.join(d, "model.jb2m")))
-    utts = refdump.load_refdump(dump)
-    feats = [synth.read_htk_param(fn)[0] for fn in files]
-    am = capi.GmmScorer(ds, mode=capi.GMM_EXACT)
-    dec = capi.Decoder(ds, am, max_utts=4, max_frames=2048)
-    for r, u in zip(dec.decode(feats), utts):
-        _check(r, u)
+def test_gpu_grammar_mode_equals_compiled_reference(extra):
+    _check_case(SweepGolden("small", extra, grammar=True))

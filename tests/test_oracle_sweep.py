@@ -1,50 +1,36 @@
-"""CPU: the restatement against the compiled reference itself (oracle/_ref/jref), across jconf options beyond the
-committed golden cases.  Runs wherever the compiled reference is present (it is built from /root/reference by
-oracle/Makefile and travels with the tree); each case pushes freshly sampled utterances through the reference and
-through the restatement and demands bit-identical state scores and an identical word trellis."""
+"""CPU: the restatement against the compiled reference across jconf options beyond the committed golden cases.  The
+reference's state scores, word trellis and pass-1 result for each case are pinned in tests/golden/sweep (written by
+tests/golden/make_golden.py from oracle/_ref/jref); the restatement must give bit-identical state scores and an
+identical word trellis."""
 import os
 
 import numpy as np
 import pytest
 
-from julius_b200 import desc, refdump, synth
-from util import ROOT, atoms_equal
+from util import GRAMMAR_SWEEP, ROOT, SWEEP, SweepGolden, atoms_equal, digest
 
 JREF = os.path.join(ROOT, "oracle", "_ref", "jref")
 
-SWEEP = [
-    ("small", ["-b", "80", "-iwcd1", "avg"]),
-    ("small", ["-b", "80", "-iwcd1", "best", "5"]),
-    ("small", ["-b", "120", "-lmp", "12.0", "-3.0"]),
-    ("small", ["-b", "200", "-bs", "60"]),                       # score-envelope pruning (SCORE_PRUNING, beam.c:2718-2730)
-    ("small", ["-multipath", "-b", "150", "-bs", "80"]),
-    ("small_sp", ["-iwsp", "-b", "100", "-bs", "50", "-iwcd1", "avg"]),
-    ("small", ["-gprune", "heuristic", "-tmix", "2", "-b", "90"]),
-    ("small_tr", ["-multipath", "-b", "90"]),                    # transparent words on the multipath tree
-    ("small_tm", ["-gprune", "none", "-b", "100"]),              # tied-mixture codebooks, calc_tied_mix.c:161-248
-    ("small_tm", ["-gprune", "safe", "-tmix", "2", "-b", "80", "-multipath"]),
-]
 
-
-GRAMMAR_SWEEP = [["-b", "100"], ["-b", "60", "-penalty1", "-2.5", "-iwcd1", "max"], ["-b", "150", "-multipath", "-penalty1", "1.5"]]
-
-
-@pytest.mark.skipif(not os.path.exists(JREF), reason="compiled reference (oracle/_ref/jref) not present")
-@pytest.mark.parametrize("extra", GRAMMAR_SWEEP, ids=[" ".join(e) for e in GRAMMAR_SWEEP])
-def test_grammar_mode_restatement_equals_compiled_reference(extra, tmp_path, oracle_lib):
-    """Grammar (DFA) recognition: category tree, category-pair constraint, insertion penalty, all sentence-initial
-    words alive at frame 0, best atom of the last frame as the pass-1 result (beam.c:1669-1760, :2404-2455, :435-458)."""
-    from oracle import fixtures
-    d = str(tmp_path)
-    m, files, dump, out = fixtures.make_fixture("small", d, n_utts=2, n_frames=180, extra_args=extra, noise_utts=1, grammar=True)
-    ds = desc.Descriptors(refdump.load_blob(os.path.join(d, "model.jb2m")))
-    assert ds.tree.lm_type == 1 and ds.tree.n_shared == 0 and ds.tree.n_init >= 1
-    for u in refdump.load_refdump(dump):
-        r = oracle_lib.beam_decode(ds, u.outprob)
+def _check_scores_and_trellis(g, oracle_lib):
+    for u, x in zip(g.utts, g.feats):
+        sc = oracle_lib.gmm_score(g.ds, x)
+        assert sc.shape == u.outprob_shape
+        assert digest(sc) == u.outprob_sha256, "state scores differ from the reference"
+        r = oracle_lib.beam_decode(g.ds, sc)           # bit-identical to the reference's own score matrix
         ok, why = atoms_equal(r["atoms"], u.atoms)
         assert ok, why
         assert r["words"] == u.words and r["status"] == u.status
-        assert np.float32(r["score"]) == np.float32(u.score)
+        assert np.float32(r["score"]) == u.score
+
+
+@pytest.mark.parametrize("extra", GRAMMAR_SWEEP, ids=[" ".join(e) for e in GRAMMAR_SWEEP])
+def test_grammar_mode_restatement_equals_compiled_reference(extra, oracle_lib):
+    """Grammar (DFA) recognition: category tree, category-pair constraint, insertion penalty, all sentence-initial
+    words alive at frame 0, best atom of the last frame as the pass-1 result (beam.c:1669-1760, :2404-2455, :435-458)."""
+    g = SweepGolden("small", extra, grammar=True)
+    assert g.ds.tree.lm_type == 1 and g.ds.tree.n_shared == 0 and g.ds.tree.n_init >= 1
+    _check_scores_and_trellis(g, oracle_lib)
 
 
 @pytest.mark.skipif(not os.path.exists(JREF), reason="compiled reference (oracle/_ref/jref) not present")
@@ -56,21 +42,6 @@ def test_tied_mixture_with_history_dependent_pruning_is_refused(tmp_path):
         fixtures.make_fixture("small_tm", str(tmp_path), n_utts=1, n_frames=50, extra_args=["-b", "60"])
 
 
-@pytest.mark.skipif(not os.path.exists(JREF), reason="compiled reference (oracle/_ref/jref) not present")
 @pytest.mark.parametrize("preset,extra", SWEEP, ids=[" ".join([p] + e) for p, e in SWEEP])
-def test_restatement_equals_compiled_reference(preset, extra, tmp_path, oracle_lib):
-    from oracle import fixtures
-    d = str(tmp_path)
-    m, files, dump, out = fixtures.make_fixture(preset, d, n_utts=1, n_frames=150, extra_args=extra, noise_utts=1)
-    ds = desc.Descriptors(refdump.load_blob(os.path.join(d, "model.jb2m")))
-    utts = refdump.load_refdump(dump)
-    assert len(utts) == len(files)
-    for u, fn in zip(utts, files):
-        x, _ = synth.read_htk_param(fn)
-        sc = oracle_lib.gmm_score(ds, x)
-        assert np.array_equal(sc.view(np.uint32), u.outprob.view(np.uint32))
-        r = oracle_lib.beam_decode(ds, u.outprob)
-        ok, why = atoms_equal(r["atoms"], u.atoms)
-        assert ok, why
-        assert r["words"] == u.words and r["status"] == u.status
-        assert np.float32(r["score"]) == np.float32(u.score)
+def test_restatement_equals_compiled_reference(preset, extra, oracle_lib):
+    _check_scores_and_trellis(SweepGolden(preset, extra), oracle_lib)

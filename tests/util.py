@@ -1,9 +1,12 @@
+import hashlib
 import json
 import os
+import re
+from types import SimpleNamespace
 
 import numpy as np
 
-from julius_b200 import desc, refdump
+from julius_b200 import desc, refdump, synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
@@ -12,6 +15,72 @@ CASES = ["tiny", "small_b100", "small_safe", "small_mp", "small_iwsp", "small_us
 DNN_CASES = ["small_dnn", "small_dnn_iwsp"]
 # pinned on the CPU only so far (the GPU suite does not run them yet)
 ORACLE_ONLY_CASES = ["small_tr", "small_tm", "small_dfa"]
+
+# jconf options beyond the golden cases above, pinned against the compiled reference in tests/golden/sweep
+SWEEP = [
+    ("small", ["-b", "80", "-iwcd1", "avg"]),
+    ("small", ["-b", "80", "-iwcd1", "best", "5"]),
+    ("small", ["-b", "120", "-lmp", "12.0", "-3.0"]),
+    ("small", ["-b", "200", "-bs", "60"]),                       # score-envelope pruning (SCORE_PRUNING, beam.c:2718-2730)
+    ("small", ["-multipath", "-b", "150", "-bs", "80"]),
+    ("small_sp", ["-iwsp", "-b", "100", "-bs", "50", "-iwcd1", "avg"]),
+    ("small", ["-gprune", "heuristic", "-tmix", "2", "-b", "90"]),
+    ("small_tr", ["-multipath", "-b", "90"]),                    # transparent words on the multipath tree
+    ("small_tm", ["-gprune", "none", "-b", "100"]),              # tied-mixture codebooks, calc_tied_mix.c:161-248
+    ("small_tm", ["-gprune", "safe", "-tmix", "2", "-b", "80", "-multipath"]),
+]
+# grammar (DFA) mode on the "small" preset
+GRAMMAR_SWEEP = [["-b", "100"], ["-b", "60", "-penalty1", "-2.5", "-iwcd1", "max"], ["-b", "150", "-multipath", "-penalty1", "1.5"]]
+# how a sweep case was sampled: utterances, noise utterances, frames (make_golden.py runs the reference on exactly these)
+SWEEP_UTTS, SWEEP_NOISE_UTTS, SWEEP_FRAMES, GRAMMAR_SWEEP_FRAMES = 2, 1, 150, 180
+
+
+def digest(a: np.ndarray) -> str:
+    """sha256 of an array's float32 bits: identical digests <=> bit-identical arrays"""
+    return hashlib.sha256(np.ascontiguousarray(a, "<f4").tobytes()).hexdigest()
+
+
+def sweep_dir(preset: str, extra: list, grammar: bool = False) -> str:
+    name = re.sub(r"[^A-Za-z0-9.]+", "_", " ".join([preset] + list(extra)).replace("-", " ")).strip("_")
+    return os.path.join(GOLDEN, "sweep", ("dfa_" if grammar else "") + name)
+
+
+def load_pinned(d: str, feats=None):
+    """meta.json and out.npz of a directory written by tests/golden/make_golden.py pin(): (meta, utterances), each
+    utterance with the reference's trellis (atoms), words, status and score, and the digest of its state scores.  With
+    feats given, every input must match the digest of the one the reference decoded."""
+    meta = json.load(open(os.path.join(d, "meta.json")))
+    out = np.load(os.path.join(d, "out.npz"))
+    assert feats is None or len(feats) == len(meta["utts"]), "the inputs are not the ones the reference decoded"
+    utts = []
+    for i, u in enumerate(meta["utts"]):
+        if feats is not None:
+            assert digest(feats[i]) == u["feats_sha256"], f"input {i} differs from the one the reference decoded"
+        utts.append(SimpleNamespace(atoms=out[f"u{i}"], words=u["words"], status=u["status"], score=np.float32(u["score"]),
+                                    outprob_shape=tuple(u["outprob_shape"]), outprob_sha256=u["outprob_sha256"]))
+    return meta, utts
+
+
+class SweepGolden:
+    """A sweep case as the compiled reference decoded it (written by tests/golden/make_golden.py).  To stay small on disk:
+    the flattened model is kept as the entries that no committed golden model holds (meta "model" maps a golden case,
+    or "" for model_delta.npz, to the entries taken from it); the inputs are regenerated from their seed and must match
+    the recorded digests; the reference's state scores are kept as digests, its trellis and pass-1 result in full."""
+
+    def __init__(self, preset: str, extra: list, grammar: bool = False):
+        from oracle import fixtures
+        d = sweep_dir(preset, extra, grammar)
+        m = synth.SynthModel(synth.SynthConfig.preset(preset))
+        self.feats = fixtures.sample_inputs(m, SWEEP_UTTS, GRAMMAR_SWEEP_FRAMES if grammar else SWEEP_FRAMES,
+                                            noise_utts=SWEEP_NOISE_UTTS, grammar=grammar)
+        self.meta, self.utts = load_pinned(d, self.feats)
+        delta = np.load(os.path.join(d, "model_delta.npz"))
+        self.blob = {}
+        for src, keys in self.meta["model"].items():
+            model = refdump.load_blob(os.path.join(GOLDEN, src, "model.jb2m")) if src else delta
+            for key in keys.split():
+                self.blob[key] = model[key]
+        self.ds = desc.Descriptors(self.blob)
 
 
 class Golden:
