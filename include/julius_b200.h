@@ -52,6 +52,12 @@ int64_t jb200_launch_count(void);
  * ---------------------------------------------------------------------------------- */
 typedef struct jb200_gmm jb200_gmm;
 
+/* The descriptor is checked before anything is uploaded: with n_gauss > 0, state_off must be non-decreasing
+ * from 0 to n_gauss (a state has at most 64 mixture slots), cd_off must be non-decreasing from 0 to n_cdset_states
+ * and every cd_states entry a state id; otherwise JB200_ERR_ARG (JB200_ERR_UNSUPPORTED for dim, -tmix, -iwcd1 best
+ * or a mixture count the kernels are not built for).  A state with no mixture slots (state_off[s] == state_off[s+1])
+ * scores LOG_ZERO, as outprob_state does for an empty mixture list.  n_gauss == 0 describes the state / cd-set layout
+ * of a DNN-HMM only: state_off may then be NULL and the state columns cannot be scored. */
 int jb200_gmm_create(const jb200_gmm_desc *desc, int device, int mode, jb200_gmm **out);
 void jb200_gmm_destroy(jb200_gmm *h);
 /* row stride (floats) of the score matrix: n_states + n_cdsets rounded up to 4 */

@@ -1,5 +1,5 @@
-// dnn_cluster.cu -- EXPERIMENTAL 2-CTA cluster variant of the DNN GEMM (JB200_DNN_KERNEL=2).  Compiled and reviewed, NOT yet
-// run on a device; kept in its own translation unit so that the shipped kernels in dnn.cu stay bit-for-bit what was
+// dnn_cluster.cu -- EXPERIMENTAL 2-CTA cluster variant of the DNN GEMM (JB200_DNN_KERNEL=2).  Opt-in (not faster than the
+// persistent kernel); held bit-identical to dnn_gemm_persistent by tests/test_gpu_scoring_shapes.py.  Kept in its own translation unit so that the shipped kernels in dnn.cu stay bit-for-bit what was
 // validated (adding a kernel to dnn.cu perturbed ptxas' register allocation of the others).  The small PTX wrappers and
 // the argument block are repeated from dnn.cu on purpose.
 #include "common.cuh"
@@ -87,7 +87,7 @@ struct PersistentCfg {
   static constexpr int SMEM = STAGES_ * STAGE + 1024 + 256;
 };
 
-// ---- 2-CTA cluster variant (EXPERIMENTAL: JB200_DNN_KERNEL=2, compiled and reviewed but not yet run on a device) -------
+// ---- 2-CTA cluster variant (EXPERIMENTAL: JB200_DNN_KERNEL=2) ------------------------------------------------------------
 // dnn_gemm_persistent<256> is bound by the TMA feed (DESIGN.md K2): ~6100 cycles for the six 128-row boxes of a stage.
 // Here two CTAs of a cluster work on vertically adjacent 128x256 tiles (same weight columns): each CTA issues its own
 // activation boxes plus HALF of the weight boxes, multicast into both CTAs' shared memory, so a stage costs four boxes

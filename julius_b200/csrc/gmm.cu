@@ -372,6 +372,25 @@ extern "C" int jb200_gmm_create(const jb200_gmm_desc *d, int device, int mode, j
     set_error("-tmix %d outside supported range 1..%d", d->gprune_num, GMM_NMAX); return JB200_ERR_UNSUPPORTED;
   }
   if (d->iwcd_method == JB200_IWCD_NBEST && d->iwcd_nbest > GMM_NMAX) { set_error("-iwcd1 best %d too large", d->iwcd_nbest); return JB200_ERR_UNSUPPORTED; }
+  // the descriptor may come from a file: every offset the packer and the kernels follow is checked here
+  if (d->n_states < 0 || d->n_gauss < 0 || d->n_cdsets < 0 || d->n_cdset_states < 0) { set_error("jb200_gmm_create: negative size"); return JB200_ERR_ARG; }
+  if (d->n_gauss > 0) {
+    if (d->dim != 39 && d->dim != 38 && d->dim != 26 && d->dim != 25) { set_error("feature dimension %d not instantiated (39, 38, 26, 25)", d->dim); return JB200_ERR_UNSUPPORTED; }
+    if (!d->state_off || !d->mean || !d->ivar || !d->gconst || !d->lnweight || !d->valid) { set_error("jb200_gmm_create: missing Gaussian arrays"); return JB200_ERR_ARG; }
+    if (d->state_off[0] != 0 || d->state_off[d->n_states] != d->n_gauss) {
+      set_error("state_off runs from %d to %d, not from 0 to n_gauss = %d", d->state_off[0], d->state_off[d->n_states], d->n_gauss); return JB200_ERR_ARG;
+    }
+    for (int s = 0; s < d->n_states; s++)
+      if (d->state_off[s + 1] < d->state_off[s]) { set_error("state_off decreases at state %d (%d -> %d)", s, d->state_off[s], d->state_off[s + 1]); return JB200_ERR_ARG; }
+  }
+  if (d->n_cdsets > 0) {
+    if (!d->cd_off || !d->cd_states) { set_error("jb200_gmm_create: missing cd-set arrays"); return JB200_ERR_ARG; }
+    if (d->cd_off[0] != 0 || d->cd_off[d->n_cdsets] != d->n_cdset_states) { set_error("cd_off does not run from 0 to n_cdset_states"); return JB200_ERR_ARG; }
+    for (int c = 0; c < d->n_cdsets; c++)
+      if (d->cd_off[c + 1] < d->cd_off[c]) { set_error("cd_off decreases at set %d", c); return JB200_ERR_ARG; }
+    for (int i = 0; i < d->n_cdset_states; i++)
+      if (d->cd_states[i] < 0 || d->cd_states[i] >= d->n_states) { set_error("cd_states[%d] = %d is not a state id", i, d->cd_states[i]); return JB200_ERR_ARG; }
+  }
   JB_CUDA(cudaSetDevice(device));
   cudaDeviceProp prop;
   JB_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -394,18 +413,24 @@ extern "C" int jb200_gmm_create(const jb200_gmm_desc *d, int device, int mode, j
     rec[rec_gconst(h->D)] = d->valid[g] ? d->gconst[g] : NAN;
     rec[rec_lnw(h->D)] = d->lnweight[g];
   }
-  // tiles: consecutive states, <= GMM_TILE_STATES states and <= GMM_TILE_GAUSS Gaussians
+  // tiles: consecutive states, <= GMM_TILE_STATES states with mixtures and <= GMM_TILE_GAUSS Gaussians.  States without
+  // mixture slots ride along in the tile of their neighbours (the kernel writes LOG_ZERO for them), so every tile
+  // stages at least one Gaussian and every state column is written
   std::vector<GmmTile> tiles;
   std::vector<int> mixcnt(h->S);
   for (int s = 0; s < h->S; s++) {
     mixcnt[s] = (h->G > 0) ? d->state_off[s + 1] - d->state_off[s] : 0;
-    if (mixcnt[s] > GMM_TILE_GAUSS) { set_error("state %d has %d mixtures (max %d)", s, mixcnt[s], GMM_TILE_GAUSS); delete h; return JB200_ERR_UNSUPPORTED; }
+    if (mixcnt[s] > GMM_TILE_GAUSS) { set_error("state %d has %d mixtures (max %d)", s, mixcnt[s], GMM_TILE_GAUSS); jb200_gmm_destroy(h); return JB200_ERR_UNSUPPORTED; }
   }
-  for (int s = 0; s < h->S;) {
-    GmmTile t{s, 0, (h->G > 0) ? d->state_off[s] : 0, 0};
-    while (s < h->S && t.ns < GMM_TILE_STATES && t.ng + mixcnt[s] <= GMM_TILE_GAUSS) { t.ng += mixcnt[s]; t.ns++; s++; }
-    if (t.ng > 0) tiles.push_back(t);
-    else if (t.ns == 0) s++;   // cannot happen (mixcnt<=TILE_GAUSS)
+  if (h->G > 0) {
+    for (int s = 0; s < h->S;) {
+      GmmTile t{s, 0, d->state_off[s], 0};
+      int filled = 0;
+      while (s < h->S && (mixcnt[s] == 0 || filled < GMM_TILE_STATES) && t.ng + mixcnt[s] <= GMM_TILE_GAUSS) {
+        filled += mixcnt[s] > 0; t.ng += mixcnt[s]; t.ns++; s++;
+      }
+      tiles.push_back(t);
+    }
   }
   h->n_tiles = (int)tiles.size();
   size_t tile_bytes = tiles.size() * sizeof(GmmTile) + mixcnt.size() * sizeof(int);

@@ -25,8 +25,23 @@ import struct
 import numpy as np
 
 SIL = "sil"
-PARMKIND_MFCC_E_D_A = 6 | 0x40 | 0x100 | 0x200  # rdparam.c / htk_param.h
+# HTK parameter kinds (libsent/include/sent/htk_param.h): base MFCC = 6, qualifiers _E 0x40, _N 0x80, _D 0x100,
+# _A 0x200, _Z 0x800
+PARMKIND_MFCC_E_D_A = 6 | 0x40 | 0x100 | 0x200
 PARMKIND_USER = 9
+# the usual MFCC layout of each feature size the GMM scorer is built for: (kind name in hmmdefs, parmKind code).
+# 25 = 12 MFCC + 12 delta + delta energy (_N drops absolute energy), the Julius dictation-kit format
+PARMKINDS = {
+    25: ("MFCC_E_D_N_Z", 6 | 0x40 | 0x100 | 0x80 | 0x800),
+    26: ("MFCC_E_D_Z", 6 | 0x40 | 0x100 | 0x800),
+    38: ("MFCC_E_D_A_N_Z", 6 | 0x40 | 0x100 | 0x200 | 0x80 | 0x800),
+    39: ("MFCC_E_D_A", PARMKIND_MFCC_E_D_A),
+}
+
+
+def parmkind_for_dim(dim: int):
+    """(hmmdefs kind name, HTK parmKind code) of a feature vector of `dim` values; USER for any other size"""
+    return PARMKINDS.get(dim, ("USER", PARMKIND_USER))
 
 
 @dataclasses.dataclass
@@ -47,11 +62,16 @@ class SynthConfig:
     sp_model: bool = False     # add a 1-state tee model "sp" (skip transition) for -iwsp; forces multipath
     transparent_words: int = 0 # the first k words get a {..} output string: transparent to the LM context (fillers)
     tied_mixture: bool = False # phonetic tied-mixture AM: one Gaussian codebook per (phone, state position), per-state weights
+    # irregular mixtures: state s has 1..n_mix mixture slots, and in a few states one slot is left out of the
+    # definition (a NULL density, rdhmmdef_mpdf.c:170-193); drawn from their own generator so the rest is unchanged
+    irregular_mix: bool = False
 
     @staticmethod
     def preset(name: str) -> "SynthConfig":
         if name == "tiny":
             return SynthConfig()
+        if name in ("tiny_d25", "tiny_d26"):   # "tiny" at the other MFCC sizes, irregular mixture counts, NULL densities
+            return SynthConfig(name=name, dim=int(name[-2:]), n_mix=6, irregular_mix=True)
         if name == "small":      # a few hundred words, used for CPU-side parity
             return SynthConfig(name="small", seed=2, n_phones=12, n_states=240, n_mix=8,
                                phys_per_phone=24, vocab=400, n_bigrams=4000,
@@ -92,6 +112,18 @@ class SynthModel:
         self.mean = (centre + rng.normal(0.0, 0.5, size=(S, M, D))).astype(np.float32)
         self.var = rng.uniform(0.3, 1.5, size=(S, M, D)).astype(np.float32)
         self.weight = rng.dirichlet(np.full(M, 2.0), size=S).astype(np.float32)
+        # ---- irregular mixtures: n_mix_of[s] slots, null[s, m] = slot left undefined (weights renormalised over the rest)
+        self.n_mix_of = np.full(S, M, dtype=np.int64)
+        self.null = np.zeros((S, M), dtype=bool)
+        if cfg.irregular_mix:
+            r2 = np.random.default_rng(cfg.seed + 1000)
+            self.n_mix_of = r2.integers(1, M + 1, size=S)
+            for s in r2.choice(S, size=S // 8, replace=False):
+                if self.n_mix_of[s] > 1:
+                    self.null[s, r2.integers(self.n_mix_of[s])] = True
+            present = (np.arange(M)[None, :] < self.n_mix_of[:, None]) & ~self.null
+            w = np.where(present, self.weight, 0.0).astype(np.float64)
+            self.weight = (w / w.sum(1, keepdims=True)).astype(np.float32)
         # ---- state pool partition by (centre phone, position)
         part = [[[] for _ in range(3)] for _ in range(P)]
         order = rng.permutation(S)
@@ -184,7 +216,7 @@ class SynthModel:
         D, M = cfg.dim, cfg.n_mix
         ln2pi = np.log(2.0 * np.pi)
         with open(path, "w") as f:
-            f.write(f"~o\n<STREAMINFO> 1 {D}\n<VECSIZE> {D}<NULLD><MFCC_E_D_A><DIAGC>\n")
+            f.write(f"~o\n<STREAMINFO> 1 {D}\n<VECSIZE> {D}<NULLD><{parmkind_for_dim(D)[0]}><DIAGC>\n")
             for name, a_self in zip(self.trans_names, self.trans_self):
                 a = np.zeros((5, 5))
                 a[0, 1] = 1.0
@@ -208,8 +240,10 @@ class SynthModel:
                     f.write(f'~s "st{s}"\n<NUMMIXES> {M}\n<TMIX> cb{int(self.book_of[s]):03d}_ ')
                     f.write(" ".join(f"{w:.8e}" for w in self.weight[s]) + "\n")
             for s in range(cfg.n_states if not cfg.tied_mixture else 0):
-                f.write(f'~s "st{s}"\n<NUMMIXES> {M}\n')
-                for m in range(M):
+                f.write(f'~s "st{s}"\n<NUMMIXES> {self.n_mix_of[s]}\n')
+                for m in range(self.n_mix_of[s]):
+                    if self.null[s, m]:
+                        continue
                     f.write(f"<MIXTURE> {m + 1} {self.weight[s, m]:.8e}\n")
                     f.write(f"<MEAN> {D}\n " + " ".join(f"{x:.8e}" for x in self.mean[s, m]) + "\n")
                     f.write(f"<VARIANCE> {D}\n " + " ".join(f"{x:.8e}" for x in self.var[s, m]) + "\n")
@@ -369,11 +403,14 @@ class SynthModel:
         return rng.normal(0.0, 1.2, size=(n_frames, self.cfg.dim)).astype(np.float32)
 
 
-def write_htk_param(path: str, feats: np.ndarray, parmkind: int = PARMKIND_MFCC_E_D_A,
+def write_htk_param(path: str, feats: np.ndarray, parmkind: int | None = None,
                     samp_period: int = 100000) -> None:
-    """Big-endian HTK parameter file (libsent/src/anlz/rdparam.c:83-187)."""
+    """Big-endian HTK parameter file (libsent/src/anlz/rdparam.c:83-187).  parmkind None: the kind the synthetic
+    hmmdefs of this feature size declare (parmkind_for_dim)."""
     feats = np.ascontiguousarray(feats, dtype=np.float32)
     T, D = feats.shape
+    if parmkind is None:
+        parmkind = parmkind_for_dim(D)[1]
     with open(path, "wb") as f:
         f.write(struct.pack(">IIHh", T, samp_period, D * 4, parmkind))
         f.write(feats.astype(">f4").tobytes())

@@ -4,7 +4,10 @@
  *   logistic table + clamp      libsent/src/phmm/calc_dnn.c:342-369
  *   calc_dnn_fma (GEMV)         libsent/src/phmm/calc_dnn_fma.c:18-95  (8 partial sums by lane,
  *                               horizontal add in lane order, + bias); scalar sub1 (calc_dnn.c:509-523)
- *                               is used when the input length is not a multiple of 8
+ *                               when the input length is not a multiple of 8.  The reference itself is no
+ *                               guide there: its FMA GEMV runs over in/8 blocks and drops the rest (its AVX
+ *                               and SSE variants refuse such layers, calc_dnn.c:395-401), so this path is
+ *                               held against float64 instead (tests/test_scoring_reference.py)
  *   dnn_calc_outprob            libsent/src/phmm/calc_dnn.c:774-868    (hidden: logistic table;
  *                               output: linear; log-softmax through addlog_array; * INV_LOG_TEN - prior)
  */

@@ -38,6 +38,10 @@ GRAMMAR_CASES = {"small_dfa"}
 CASES = {
     # name: (preset, n_utts, n_frames, noise_utts, extra args)
     "tiny": ("tiny", 2, 150, 0, []),
+    # the other MFCC sizes the GMM scorer is built for (25 = MFCC_E_D_N_Z, 26 = MFCC_E_D_Z), 1..6 mixtures per state and
+    # a few NULL densities
+    "tiny_d25": ("tiny_d25", 2, 150, 0, []),
+    "tiny_d26": ("tiny_d26", 2, 150, 0, []),
     "small_b100": ("small", 2, 200, 1, ["-b", "100"]),
     "small_safe": ("small", 1, 150, 0, ["-gprune", "safe", "-tmix", "2", "-b", "60", "-iwcd1", "max"]),
     # multipath tree (non-emitting word-begin/word-end nodes), beam.c:2752-2828
@@ -61,6 +65,11 @@ DNN_CASES = {
     # configs[4] flavour: DNN-HMM on a multipath tree with -iwsp and a wide beam
     "small_dnn_iwsp": ("small_sp", dict(in_dim=120, feature_len=40, context_len=3, hidden=128, layers=3), 2, 150,
                        ["-iwsp", "-iwcd1", "max", "-b", "600"]),
+    # widths off the GPU kernel's tiles: 112 inputs, 104 hidden (ends inside a 32-column epilogue chunk), 60 outputs (not a
+    # multiple of 4).  Widths that are not multiples of 8 cannot be pinned here: the reference's x86 FMA GEMV
+    # (calc_dnn_fma.c:18-95) runs over in/8 blocks of 8 and silently drops the remainder, its AVX and SSE variants refuse
+    # such layers (calc_dnn.c:395-401).  tests/test_scoring_reference.py checks them against float64 instead.
+    "tiny_dnn_odd": ("tiny", dict(in_dim=112, feature_len=28, context_len=4, hidden=104, layers=2), 2, 150, ["-b", "150"]),
 }
 
 

@@ -11,8 +11,10 @@ from julius_b200 import desc, refdump, synth
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 # small_userlm: user-defined LM functions (-userlm) on top of the N-gram, tabulated by the exporter
-CASES = ["tiny", "small_b100", "small_safe", "small_mp", "small_iwsp", "small_userlm"]
-DNN_CASES = ["small_dnn", "small_dnn_iwsp"]
+# tiny_d25 / tiny_d26: 25- and 26-dimensional features (MFCC_E_D_N_Z, MFCC_E_D_Z), 1..6 mixtures per state, NULL densities
+CASES = ["tiny", "small_b100", "small_safe", "small_mp", "small_iwsp", "small_userlm", "tiny_d25", "tiny_d26"]
+# tiny_dnn_odd: 117 -> 100 x 2 -> 60, widths that are not multiples of 8 (and an output width not a multiple of 4)
+DNN_CASES = ["small_dnn", "small_dnn_iwsp", "tiny_dnn_odd"]
 # pinned on the CPU only so far (the GPU suite does not run them yet)
 ORACLE_ONLY_CASES = ["small_tr", "small_tm", "small_dfa"]
 
@@ -131,4 +133,66 @@ def full_dnn_blob(seed=3, in_dim=528, hidden=2048, layers=7, n_out=3000):
         b[f"dnn.l{i}.b"] = (rng.standard_normal(dims[i + 1]) * 0.1).astype(np.float32)
     prior = rng.dirichlet(np.full(n_out, 5.0))
     b["dnn.state_prior"] = np.log10(prior).astype(np.float32)
+    return b
+
+
+LOG_ZERO = np.float32(-1000000.0)
+
+
+def gmm_blob(dim, counts, seed=0, null_states=(), null_gauss=(), gprune=(0, 0), cdsets=None, iwcd=(2, 3)):
+    """A synthetic GMM acoustic model as a flattened-model blob dict (the layout the export plugin writes): state s has
+    counts[s] mixture slots (0 allowed); every slot of the states in null_states, and the global slots in null_gauss,
+    are NULL densities (valid 0, ln weight LOG_ZERO, as the reference reads an undefined <MIXTURE>,
+    rdhmmdef_mpdf.c:170-193).  Means N(0,1), variances U(0.3,1.5), Dirichlet(2) weights, gconst = D ln 2pi + sum ln var.
+    gprune = (method, -tmix); cdsets = list of state-id lists (pseudo-phone sets); iwcd = (method, N)."""
+    rng = np.random.default_rng(seed)
+    counts = np.asarray(counts, np.int64)
+    S, G = len(counts), int(counts.sum())
+    off = np.zeros(S + 1, np.int32)
+    off[1:] = np.cumsum(counts)
+    var = rng.uniform(0.3, 1.5, size=(G, dim))
+    valid = np.ones(G, np.uint8)
+    lnw = np.zeros(G, np.float32)
+    for s in range(S):
+        if counts[s]:
+            lnw[off[s]:off[s + 1]] = np.log(rng.dirichlet(np.full(counts[s], 2.0)))
+        if s in null_states:
+            valid[off[s]:off[s + 1]] = 0
+    valid[list(null_gauss)] = 0
+    lnw[valid == 0] = LOG_ZERO
+    b = {"gmm.n_states": np.array([S], np.int32), "gmm.dim": np.array([dim], np.int32),
+         "gmm.n_gauss": np.array([G], np.int32), "gmm.max_mix": np.array([max(1, int(counts.max()))], np.int32),
+         "gmm.gprune_method": np.array([gprune[0]], np.int32), "gmm.gprune_num": np.array([gprune[1]], np.int32),
+         "gmm.state_off": off, "gmm.mean": rng.standard_normal((G, dim)).astype(np.float32).ravel(),
+         "gmm.ivar": (1.0 / var).astype(np.float32).ravel(),
+         "gmm.gconst": (dim * np.log(2 * np.pi) + np.log(var).sum(1)).astype(np.float32),
+         "gmm.lnweight": lnw, "gmm.valid": valid,
+         "am.iwcd_method": np.array([iwcd[0]], np.int32), "am.iwcd_nbest": np.array([iwcd[1]], np.int32)}
+    if cdsets is not None:
+        b["am.n_cdsets"] = np.array([len(cdsets)], np.int32)
+        b["am.cd_off"] = np.concatenate([[0], np.cumsum([len(c) for c in cdsets])]).astype(np.int32)
+        b["am.cd_states"] = np.concatenate([np.asarray(c, np.int32) for c in cdsets]).astype(np.int32)
+        b["am.n_cdset_states"] = np.array([len(b["am.cd_states"])], np.int32)
+    return b
+
+
+def gmm_frames(blob, T, seed=1):
+    """T feature vectors, each drawn around the mean of a random Gaussian of the model (so that every state scores over
+    a wide range, near and far), with one in eight frames far from every mean."""
+    rng = np.random.default_rng(seed)
+    D = int(blob["gmm.dim"][0])
+    mean = blob["gmm.mean"].reshape(-1, D)
+    x = mean[rng.integers(len(mean), size=T)] + rng.normal(0.0, 0.7, size=(T, D))
+    far = rng.random(T) < 0.125
+    x[far] = rng.normal(0.0, 4.0, size=(int(far.sum()), D))
+    return x.astype(np.float32)
+
+
+def dnn_blob(in_dim, hidden, layers, out_dim, seed=7, w_scale=1.5):
+    """A random-init DNN (full_dnn_blob's initialisation) with `layers` hidden layers of width `hidden`; layers == 0
+    gives a one-layer network whose first layer is the output layer."""
+    b = full_dnn_blob(seed=seed, in_dim=in_dim, hidden=hidden, layers=layers, n_out=out_dim)
+    if w_scale != 1.5:
+        for i in range(layers):
+            b[f"dnn.l{i}.w"] = (b[f"dnn.l{i}.w"] * np.float32(w_scale / 1.5)).astype(np.float32)
     return b
